@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """Benchmark of the SIFT hot path on B200 (contract in the task description / SURVEY.md 8d).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...          (one rank per GPU, no data-path collective)
+
+--dump-outputs DIR writes the features and descriptors the `value` path returned in its last timed step as .npy files
+(dump_outputs), so that two builds can be compared output for output on the same seeded frames.
 
 Workload ("step") = one pass of the hot path over a batch of FRAMES_PER_STEP synthetic 3840x2160
 8-bit frames per GPU, popsift::Config defaults with octaves=5, levels=3 (BASELINE.json configs[2]:
@@ -249,23 +252,34 @@ def run_ours(args, rank, world, local_rank):
         if rc != 0:
             raise SystemExit("popsift_b200 error %d: %s" % (rc, L.ps_last_error(ctx).decode()))
 
-    def step_dev():
-        """FRAMES_PER_STEP frames, SLOTS in flight; every job's features + descriptors land on the host."""
+    def step_dev(keep=None):
+        """FRAMES_PER_STEP frames, SLOTS in flight; every job's features + descriptors land on the host.
+        `keep`: a _PinnedBlock with room for the whole step; each frame's results then land in a region of their own,
+        appended to keep.frames as (first feature, features, first descriptor, descriptors)."""
         tot_f = tot_d = 0
         inflight = []
+
+        def fetch(s0):
+            chk(L.ps_counts(ctx, s0, C.byref(nf), C.byref(nd)))
+            if keep is None:
+                chk(L.ps_download(ctx, s0, feat_buf.ctypes.data, desc_buf.ctypes.data))
+            else:
+                if tot_f + nf.value > keep.n_feat or tot_d + nd.value > keep.n_desc:
+                    raise SystemExit("bench.py: the last timed step returned more results than the warm-up step")
+                chk(L.ps_download(ctx, s0, keep.pf + 72 * tot_f, keep.pd + 512 * tot_d))
+                keep.frames.append((tot_f, nf.value, tot_d, nd.value))
+            return nf.value, nd.value
+
         for i, df in enumerate(dev_frames):
             s = i % SLOTS
             if len(inflight) == SLOTS:
-                s0 = inflight.pop(0)
-                chk(L.ps_counts(ctx, s0, C.byref(nf), C.byref(nd)))
-                chk(L.ps_download(ctx, s0, feat_buf.ctypes.data, desc_buf.ctypes.data))
-                tot_f += nf.value; tot_d += nd.value
+                f, d = fetch(inflight.pop(0))
+                tot_f += f; tot_d += d
             chk(L.ps_submit_dev_u8(ctx, s, df.data_ptr(), W, W, H))
             inflight.append(s)
         for s0 in inflight:
-            chk(L.ps_counts(ctx, s0, C.byref(nf), C.byref(nd)))
-            chk(L.ps_download(ctx, s0, feat_buf.ctypes.data, desc_buf.ctypes.data))
-            tot_f += nf.value; tot_d += nd.value
+            f, d = fetch(s0)
+            tot_f += f; tot_d += d
         return tot_f, tot_d
 
     def barrier():
@@ -278,7 +292,13 @@ def run_ours(args, rank, world, local_rank):
     if rank == 0:
         sampler.start()
     for _ in range(args.warmup):
-        step_dev()
+        warm = step_dev()
+    last_step = None
+    if args.dump_outputs and rank == 0:
+        # the last timed step downloads into a block allocated here, one region per frame, so that keeping its results
+        # changes only where ps_download writes; sized from the warm-up step, which ran the same frames
+        last_step = api._PinnedBlock(L, warm[0] + warm[0] // 8 + 1, warm[1] + warm[1] // 8 + 1)
+        last_step.frames = []
     barrier()
     launches0 = L.ps_launch_count(ctx)
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -291,8 +311,8 @@ def run_ours(args, rank, world, local_rank):
     t0 = time.perf_counter()
     wall0 = time.time()
     counts = (0, 0)
-    for _ in range(args.steps):
-        counts = step_dev()
+    for k in range(args.steps):
+        counts = step_dev(last_step if k == args.steps - 1 else None)
     for st in slot_streams:        # ev1 after everything the slots did
         e = torch.cuda.Event()
         e.record(st)
@@ -303,6 +323,10 @@ def run_ours(args, rank, world, local_rank):
     dev_ms = ev0.elapsed_time(ev1)
     launches = L.ps_launch_count(ctx) - launches0
     clocks = sampler.stop(wall0, time.time()) if rank == 0 else None
+    if last_step is not None:
+        dump_outputs(args.dump_outputs, [(last_step.feat[f0:f0 + n], last_step.desc[d0:d0 + m], last_step.pd + 512 * d0)
+                                         for f0, n, d0, m in last_step.frames])
+        last_step.free()
 
     # ---------------- roofline of the pyramid stage (same context, slot 0 holds the last frame) ----
     chk(L.ps_submit_dev_u8(ctx, 0, dev_frames[0].data_ptr(), W, W, H))
@@ -355,10 +379,10 @@ def run_ours(args, rank, world, local_rank):
         step_e2e()
     barrier()
     t0 = time.perf_counter()
-    for _ in range(max(2, args.steps // 2)):
+    for _ in range(args.steps):
         step_e2e()
     barrier()
-    pinned_wall_ms = (time.perf_counter() - t0) * 1e3 / max(2, args.steps // 2)
+    pinned_wall_ms = (time.perf_counter() - t0) * 1e3 / args.steps
     ps.uninit()
     del pinned
 
@@ -428,6 +452,51 @@ def run_ours(args, rank, world, local_rank):
     if world == 1:      # reported baselines: rank 0 at N=1 only (torchrun pins OMP_NUM_THREADS=1)
         out.update(cpu_baselines(frames))
     return out
+
+
+DUMP_BYTES = 64 << 20
+DUMP_DESC_SAMPLE = 65536
+
+
+def dump_outputs(out_dir, per_frame, seed=0):
+    """What the timed (device-resident) path handed back for each frame of its last step, as .npy files in `out_dir`.
+    The library emits features in no fixed order, so each frame's features are sorted (octave, y, x, sigma, num_ori,
+    orientations) and orientation slots beyond num_ori are written as 0:
+      counts.npy           float64 [frames, 2]   features, descriptors per frame
+      features.npy         float32 [n, 10]       frame, octave, x, y, sigma, num_ori, ori[4]
+      descriptors.npy      float32 [s, 128]      a seeded sample of the descriptors (all of them if they fit 64 MB)
+      descriptor_rows.npy  float64 [s, 2]        row in features.npy and orientation index of each sampled descriptor
+    Descriptor j of the full list is the one of feature row r, orientation k, enumerated in row order, then k.
+    `per_frame`: (features, descriptors, host address of descriptor 0 that the features' desc_ptr refer to) per frame."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts, feats, rows, idx = [], [], [], []
+    for i, (feat, desc, desc_base) in enumerate(per_frame):
+        n = feat["num_ori"].astype(np.int64)
+        ori = np.where(np.arange(4)[None, :] < n[:, None], feat["ori"], np.float32(0))
+        order = np.lexsort(tuple(ori[:, k] for k in range(3, -1, -1)) + (n, feat["sigma"], feat["x"], feat["y"], feat["octave"]))
+        t = np.zeros((len(feat), 10), np.float32)
+        t[:, 0] = i
+        t[:, 1:6] = np.stack([feat["octave"], feat["x"], feat["y"], feat["sigma"], n], 1)[order]
+        t[:, 6:] = ori[order]
+        base = sum(len(f) for f in feats)
+        nk = n[order]
+        k = np.arange(nk.sum()) - np.repeat(np.cumsum(nk) - nk, nk)
+        f_in = np.repeat(order, nk)
+        rows.append(np.stack([base + np.repeat(np.arange(len(order)), nk), k], 1))
+        idx.append(np.stack([np.full(len(k), i), (feat["desc_ptr"][f_in, k].astype(np.int64) - desc_base) // 512], 1))
+        counts.append((len(feat), len(desc)))
+        feats.append(t)
+    features = np.concatenate(feats) if feats else np.zeros((0, 10), np.float32)
+    rows, idx = np.concatenate(rows), np.concatenate(idx)
+    room = max(0, (DUMP_BYTES - features.nbytes - 16 * len(counts)) // (512 + 16))
+    pick = np.arange(len(rows))
+    if len(rows) > min(room, DUMP_DESC_SAMPLE):
+        pick = np.sort(np.random.default_rng(seed).choice(len(rows), min(room, DUMP_DESC_SAMPLE), replace=False))
+    desc = np.stack([per_frame[f][1][d] for f, d in idx[pick]]) if len(pick) else np.zeros((0, 128), np.float32)
+    np.save(os.path.join(out_dir, "counts.npy"), np.array(counts, np.float64).reshape(-1, 2))
+    np.save(os.path.join(out_dir, "features.npy"), features)
+    np.save(os.path.join(out_dir, "descriptors.npy"), desc.astype(np.float32))
+    np.save(os.path.join(out_dir, "descriptor_rows.npy"), rows[pick].astype(np.float64))
 
 
 def cpu_baselines(frames, n_oracle=4):
@@ -520,7 +589,13 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path computed in its last step (rank 0's frames) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -202,6 +202,11 @@ def read_ref_features(path: str, with_rev: bool = False):
     return feat, desc, rev
 
 
+def run_key(w: int, h: int, seed: int, args) -> str:
+    """key of a reference run on make_frame(w, h, seed) with these ref_dump arguments in tests/golden/ref_runs.json"""
+    return "%dx%d_s%d %s" % (w, h, seed, " ".join(args))
+
+
 def flatten(feat, desc):
     """-> array [n_desc, 4] of (x, y, sigma, theta) and the matching descriptors, one row per
     (feature, orientation)."""
