@@ -166,7 +166,11 @@ const char* ps_last_error(const ps_ctx* ctx);
 int ps_submit_u8 (ps_ctx* ctx, int slot, const uint8_t* host_img, int w, int h);
 /* float images, value range [0,1) (reference popsift.h:62-69, s_image.cu:262-291) */
 int ps_submit_f32(ps_ctx* ctx, int slot, const float* host_img, int w, int h);
-/* same, input already resident in device memory (pitch in bytes); no host copy */
+/* same, input already resident in device memory of the context's device, `pitch` bytes from one row to the
+ * next (pitch >= w, else PS_ERR_ARG); no host copy.  The image is copied device to device on the slot's
+ * stream, which is NOT ordered after the caller's streams: the image must be complete when the call is
+ * made (synchronize the stream that wrote it first).  `dev_img` is read asynchronously: it must stay valid
+ * and unmodified until ps_wait_input(), ps_counts() or ps_sync() has returned for this slot. */
 int ps_submit_dev_u8(ps_ctx* ctx, int slot, const uint8_t* dev_img, size_t pitch, int w, int h);
 
 /* replaces Pyramid::readDescCountersFromDevice (reference sift_pyramid.cu:371-379):
@@ -203,8 +207,9 @@ int ps_match(int device, const ps_descriptor* d_left, int n_left, const ps_descr
  * buffers are staged through the slot's own pinned buffers (one extra host memcpy). */
 void* ps_host_alloc(size_t bytes);
 void  ps_host_free(void* p);
-/* waits until the input image of the slot's last ps_submit_* has been consumed (its host -> device copy
- * is complete): after this a page-locked input buffer may be reused.  Does not wait for the kernels. */
+/* waits until the input image of the slot's last ps_submit_* has been consumed (its copy into the slot's
+ * own image buffer is complete): after this a page-locked host buffer or a ps_submit_dev_u8 device buffer
+ * may be reused.  Does not wait for the kernels. */
 int ps_wait_input(ps_ctx* ctx, int slot);
 /* waits for the slot's stream without reading anything */
 int ps_sync(ps_ctx* ctx, int slot);

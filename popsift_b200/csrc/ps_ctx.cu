@@ -60,7 +60,7 @@ struct Slot {
     ps_descriptor* h_desc = nullptr;  size_t h_desc_cap = 0;
     cudaEvent_t ev[PS_NUM_STAGES + 1] = {};
     cudaEvent_t done = nullptr;
-    cudaEvent_t in_done = nullptr;   // recorded after the host -> device copy of the slot's input image
+    cudaEvent_t in_done = nullptr;   // recorded after the copy of the slot's input image (host or device source)
     bool in_pending = false;         // in_done has been recorded at least once
     int ext_cap = 0, desc_cap = 0;   // capacity of d_ext / d_feat and of d_desc / d_f2e; grown on demand (regrow_slot)
     // the slot's per-frame work as a CUDA graph (submit_common)
@@ -727,14 +727,19 @@ extern "C" int ps_submit_dev_u8(ps_ctx* ctx, int slot, const uint8_t* dev_img, s
 {
     Slot* s = get_slot(ctx, slot);
     if (!s || !dev_img) return ctx ? ctx->fail(PS_ERR_ARG, "ps_submit_dev_u8: bad argument") : PS_ERR_ARG;
-    if (w < 1 || h < 1 || w > ctx->max_w || h > ctx->max_h || pitch < (size_t)w)
+    if (w < 1 || h < 1 || w > ctx->max_w || h > ctx->max_h)
         return ctx->fail(PS_ERR_TOO_LARGE, "image %dx%d exceeds context maximum %dx%d", w, h, ctx->max_w, ctx->max_h);
+    if (pitch < (size_t)w)
+        return ctx->fail(PS_ERR_ARG, "ps_submit_dev_u8: pitch %zu is smaller than the image width %d", pitch, w);
     PS_CUDA(ctx, cudaSetDevice(ctx->device));
     int rc = build_view(ctx, *s, w, h);
     if (rc != PS_OK) return rc;
     s->is_float = false;
     if (ctx->timing) PS_CUDA(ctx, cudaEventRecord(s->ev[0], s->stream));
     PS_CUDA(ctx, cudaMemcpy2DAsync(s->d_img, u8_pitch(w), dev_img, pitch, (size_t)w, (size_t)h, cudaMemcpyDeviceToDevice, s->stream));
+    // ps_wait_input: the caller may overwrite dev_img once this copy has left it
+    PS_CUDA(ctx, cudaEventRecord(s->in_done, s->stream));
+    s->in_pending = true;
     return submit_common(ctx, *s);
 }
 
