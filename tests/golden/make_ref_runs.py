@@ -11,6 +11,7 @@ Fixtures:
                       affine set computed from the reference's full outputs
   ref_runs_desc.npz   per run with a descriptor sample: <key>|keys [k, 5] (octave, x, y, sigma, theta) and <key>|desc
                       [k, 128], drawn by compare.descriptor_sample (seed 0)
+  feat_<name>.npz     the full features (feat, in ref_dump's record layout) and descriptors (desc) of the FULL_F256 runs
 """
 import glob
 import hashlib
@@ -63,7 +64,35 @@ RUNS = [
     (640, 480, 37, ["--log", "--mode", "vlfeat", "--norm", "classic", "--gauss-mode", "fixed15"], SAMPLE),
     # test_direct_scaling_with_every_gauss_mode
 ] + [(512, 384, 39, ["--log", "--mode", "vlfeat", "--norm", "classic", "--gauss-mode", g, "--direct-scaling"], 0)
-     for g in ("relative", "fixed9", "fixed15", "vlfeat-direct")]
+     for g in ("relative", "fixed9", "fixed15", "vlfeat-direct")] + [
+    # tests/test_config_settings.py: threshold (OpenCV mode floors the peak threshold: 0.02 -> 0, 0.05 -> 2), edge limit,
+    # initial blur (above the level-0 sigma at 1.0 with the default up-scale; 0 = no assumed blur), normalization multiplier
+    (640, 480, 3, ["--mode", "vlfeat", "--norm", "classic", "--threshold", "0"], SAMPLE),
+    (640, 480, 3, ["--mode", "opencv", "--norm", "classic", "--threshold", "0.02"], SAMPLE),
+    (640, 480, 3, ["--mode", "opencv", "--threshold", "0.05"], SAMPLE),
+    (640, 480, 3, ["--mode", "popsift", "--threshold", "0.5"], SAMPLE),
+] + [(640, 480, 3, ["--mode", "vlfeat", "--norm", "classic", "--edge-limit", x], SAMPLE) for x in ("0", "2.5", "50")] + [
+    (640, 480, 5, ["--log", "--initial-blur", "0"], SAMPLE),
+    (640, 480, 5, ["--log", "--initial-blur", "1.0"], SAMPLE),
+    (640, 480, 5, ["--log", "--initial-blur", "0.3", "--downsampling", "0"], SAMPLE),
+    (640, 480, 5, ["--log", "--initial-blur", "1.0", "--direct-scaling", "--mode", "vlfeat", "--norm", "classic"], SAMPLE),
+    (640, 480, 5, ["--log", "--initial-blur", "1.0", "--gauss-mode", "vlfeat-direct", "--mode", "vlfeat", "--norm", "classic"], SAMPLE),
+    (640, 480, 5, ["--log", "--initial-blur", "0", "--gauss-mode", "relative", "--mode", "vlfeat", "--norm", "classic"], SAMPLE),
+    (640, 480, 1, ["--norm-multi", "9"], SAMPLE),
+    (640, 480, 1, ["--norm", "classic", "--norm-multi", "9"], SAMPLE),
+    (640, 480, 1, ["--norm-multi", "-3"], SAMPLE),
+    (640, 480, 1, ["--desc-mode", "grid", "--norm-multi", "9"], SAMPLE),
+]
+
+# (name, ref_dump arguments) of the runs on make_frame(256, 192, 3) whose features and descriptors are kept in full as
+# feat_<name>.npz (tests/test_oracle_golden.py::test_features_vs_reference)
+FULL_F256 = [
+    ("f256_threshold0", ["--mode", "vlfeat", "--norm", "classic", "--threshold", "0"]),
+    ("f256_opencv_threshold002", ["--mode", "opencv", "--norm", "classic", "--threshold", "0.02"]),
+    ("f256_edge_limit2_5", ["--mode", "vlfeat", "--norm", "classic", "--edge-limit", "2.5"]),
+    ("f256_initial_blur1", ["--initial-blur", "1.0"]),
+    ("f256_norm_multi9", ["--norm-multi", "9"]),
+]
 
 
 def record(out_bin, k, logdir=None):
@@ -87,6 +116,7 @@ def record(out_bin, k, logdir=None):
 
 def main(out_dir):
     assert os.path.exists(REF), "build the reference first: make -C oracle ref"
+    os.makedirs(out_dir, exist_ok=True)
     runs, samples = {}, {}
 
     def keep(key, rec, sample):
@@ -103,6 +133,13 @@ def main(out_dir):
             subprocess.run([REF, "-i", "f.pgm", "-o", "f.bin"] + args, cwd=wd, check=True, capture_output=True)
             rec, sample, _ = record(os.path.join(wd, "f.bin"), k, wd if "--log" in args else None)
             keep(ol.run_key(w, h, seed, args), rec, sample)
+        write_pgm(os.path.join(td, "f256.pgm"), make_frame(256, 192, 3))
+        for name, args in FULL_F256:
+            out = os.path.join(td, name + ".bin")
+            subprocess.run([REF, "-i", os.path.join(td, "f256.pgm"), "-o", out] + args, check=True, capture_output=True)
+            feat, desc = ol.read_ref_features(out)
+            np.savez_compressed(os.path.join(out_dir, "feat_%s.npz" % name), feat=feat, desc=desc.astype(np.float32))
+            print(name, [len(feat), len(desc)], flush=True)
         # test_affine_set_per_keypoint_diff_and_repeatability: the six images of the affine set, VLFeat mode
         aset, full = affine_set(), []
         for i, (im, _) in enumerate(aset, 1):
@@ -125,7 +162,6 @@ def main(out_dir):
         for i in range(32):
             rec, sample, _ = record(os.path.join(td, "bench.%d" % i), 1)
             keep("bench%d %s" % (i, " ".join(args)), rec, sample)
-    os.makedirs(out_dir, exist_ok=True)
     with open(os.path.join(out_dir, "ref_runs.json"), "w") as fh:       # one run per line
         fh.write("{\n%s\n}\n" % ",\n".join("%s: %s" % (json.dumps(k), json.dumps(runs[k], sort_keys=True)) for k in sorted(runs)))
     np.savez_compressed(os.path.join(out_dir, "ref_runs_desc.npz"), **samples)

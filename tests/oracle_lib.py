@@ -97,6 +97,9 @@ def make_config(**kw) -> OrcConfig:
             c.norm_mode = NORM[v]
         elif k == "downsampling":
             c.upscale = -float(v)
+        elif k == "initial_blur":
+            c.initial_blur = float(v)
+            c.has_initial_blur = int(v != 0.0)          # Config::setInitialBlur (reference sift_conf.cu:246-255)
         else:
             assert hasattr(c, k), k
             setattr(c, k, v)
