@@ -387,8 +387,10 @@ __device__ __forceinline__ void stage3(const PyramidView& pyr, const Consts& k, 
     }
 }
 
-template <int MODE, int CTAS>
-__global__ void __launch_bounds__(kScanThreads, CTAS)
+// 3 resident CTAs per SM: 80 registers, 77.7 us per 4K frame; 4 CTAs force 64 registers, which spill in the
+// candidate loop (84.4 us)
+template <int MODE>
+__global__ void __launch_bounds__(kScanThreads, 3)
 cand_extrema_kernel(PyramidView pyr, Consts k, InitialExtremum* __restrict__ iext, Counters* ct)
 {
     __shared__ Q2Entry q2[kScanThreads / 32][kQ2];
@@ -514,11 +516,7 @@ template <int MODE>
 int launch_scan(const PyramidView& pyr, const Consts& k, InitialExtremum* iext, Counters* ct, cudaStream_t st)
 {
     if (pyr.cands_filled && !dense_choice()) {
-        // resident CTAs per SM: 3 (80 registers: 77.7 us per 4K frame) or 4 (64 registers, spills in the candidate loop:
-        // 84.4 us); POPSIFT_B200_EXTREMA_CTAS=4 for A/B timing
-        static const int ctas = [] { const char* e = getenv("POPSIFT_B200_EXTREMA_CTAS"); return e && atoi(e) == 4 ? 4 : 3; }();
-        if (ctas == 3) cand_extrema_kernel<MODE, 3><<<sm_count() * 3, kScanThreads, 0, st>>>(pyr, k, iext, ct);
-        else           cand_extrema_kernel<MODE, 4><<<sm_count() * 4, kScanThreads, 0, st>>>(pyr, k, iext, ct);
+        cand_extrema_kernel<MODE><<<sm_count() * 3, kScanThreads, 0, st>>>(pyr, k, iext, ct);
         return 1;
     }
     int launches = 0;

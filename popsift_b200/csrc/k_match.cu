@@ -12,10 +12,9 @@
 //                             descriptor.  Three tf32 products hi.hi + hi.lo + lo.hi give a.b to ~2^-21 relative.
 //   2. match_tc_kernel        one CTA per 128 left descriptors.  The A tile (hi and lo, 128 x 128 floats each) is
 //                             loaded once with TMA (SWIZZLE_128B, K-major) and stays in shared memory; the right
-//                             descriptors stream through a 4-stage TMA ring of [64 descriptors x 32 floats] tiles (hi and lo),
-//                             every CTA starting at a different tile of the right set; ONE thread
-//                             issues tcgen05.mma.kind::tf32 (M = 128, N = 64, K = 8) into a double-buffered fp32
-//                             accumulator in TMEM; four epilogue warps read the accumulator with tcgen05.ld
+//                             descriptors stream in order through a 2-stage TMA ring of [128 descriptors x 32 floats]
+//                             tiles (hi and lo); ONE thread issues tcgen05.mma.kind::tf32 (M = 128, N = 128, K = 8) into
+//                             a double-buffered fp32 accumulator in TMEM; four epilogue warps read the accumulator with tcgen05.ld
 //                             (thread = one left descriptor = one TMEM lane) and keep that descriptor's four best
 //                             candidates |b|^2 - 2 a.b in registers.  The n_left x n_right distance matrix never
 //                             touches HBM.  Warp roles: 0 = TMA producer, 1 = MMA issuer + TMEM owner, 2..5 = epilogue.
@@ -31,8 +30,6 @@
 #include "tma_util.h"
 
 #include <cstdint>
-#include <cstdlib>
-#include <cstring>
 #include <mutex>
 
 namespace psb {
@@ -124,9 +121,11 @@ constexpr int KB = 32;                       // floats per K-block = one 128-byt
 constexpr int NKB = 128 / KB;                // K-blocks per descriptor
 constexpr int UMMA_K = 8;                    // tf32: 32 bytes per instruction
 constexpr int TILE_BYTES = BM * KB * 4;      // 16 KB: one [128 rows x 128 bytes] operand tile of the left set
+constexpr int BTILE_BYTES = BN * KB * 4;     // 16 KB: one [128 rows x 128 bytes] operand tile of the right set
+constexpr int STAGES = 2;                    // B ring: stages of [hi, lo] tiles
 constexpr int TC_THREADS = 192;              // 6 warps
 constexpr int kCand = 4;                     // candidates kept per left descriptor
-constexpr size_t TC_SMEM = (size_t)2 * NKB * TILE_BYTES + 64 * 1024;    // A hi/lo resident + 64 KB B ring = 192 KB
+constexpr size_t TC_SMEM = (size_t)2 * NKB * TILE_BYTES + (size_t)STAGES * 2 * BTILE_BYTES;   // A hi/lo resident + 64 KB B ring = 192 KB
 constexpr int TMEM_COLS = 2 * BN;            // two fp32 accumulators of 128 columns
 
 __device__ __forceinline__ unsigned s32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -155,7 +154,7 @@ __device__ __forceinline__ uint64_t umma_desc(const void* tile)
     return (uint64_t)((s32(tile) >> 4) & 0x3fffu) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
 }
 // cute::UMMA::InstrDescriptor: D = F32 (1 << 4), A = B = TF32 (2 << 7, 2 << 10), both K-major, N >> 3 at [17,23), M >> 4 at [24,29)
-__host__ __device__ constexpr unsigned idesc_for(int n) { return (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(n >> 3) << 17) | ((unsigned)(BM >> 4) << 24); }
+constexpr unsigned kIdesc = (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(BN >> 3) << 17) | ((unsigned)(BM >> 4) << 24);
 
 __device__ __forceinline__ void umma_tf32(unsigned d_tmem, uint64_t a_desc, uint64_t b_desc, unsigned accumulate, unsigned kIdesc)
 {
@@ -231,28 +230,13 @@ __device__ __forceinline__ void top4_group(Top4& T, const unsigned (&r)[32], con
     }
 }
 
-// Every CTA walks the right set from a different tile, so that the CTAs do not all pull the same lines out of the same L2
-// slices at the same moment (the candidate selection does not depend on the order of the tiles)
-template <bool ROT>
-__device__ __forceinline__ int tile_of(int j, int n_tiles)
-{
-    if (!ROT) return j;
-    const int t = j + (int)((blockIdx.x * 37u) % (unsigned)n_tiles);
-    return t >= n_tiles ? t - n_tiles : t;
-}
-
-// BNS = right descriptors per stage of the B ring and N of one MMA (128: two 32 KB stages; 64: four 16 KB stages)
-template <int BNS, bool ROT>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 match_tc_kernel(const __grid_constant__ CUtensorMap tm_lhi, const __grid_constant__ CUtensorMap tm_llo,
                 const __grid_constant__ CUtensorMap tm_rhi, const __grid_constant__ CUtensorMap tm_rlo,
                 const float* __restrict__ rnorm, int nl, int n_tiles, int32_t* __restrict__ cand)
 {
-    constexpr int BTILE_BYTES = BNS * KB * 4;                   // one [BNS rows x 128 bytes] operand tile of the right set
-    constexpr int STAGES = 64 * 1024 / (2 * BTILE_BYTES);
-    constexpr unsigned kIdesc = idesc_for(BNS);
     extern __shared__ __align__(1024) uint8_t smem[];          // SWIZZLE_128B tiles: 1024-byte aligned
-    __shared__ __align__(8) uint64_t a_full, b_full[4], b_empty[4], acc_full[2], acc_empty[2];
+    __shared__ __align__(8) uint64_t a_full, b_full[STAGES], b_empty[STAGES], acc_full[2], acc_empty[2];
     __shared__ unsigned tmem_base_s;
     uint8_t* A_hi = smem;                                       // NKB tiles
     uint8_t* A_lo = smem + NKB * TILE_BYTES;
@@ -284,17 +268,14 @@ match_tc_kernel(const __grid_constant__ CUtensorMap tm_lhi, const __grid_constan
                 tma_tile(A_lo + kb * TILE_BYTES, &tm_llo, kb * KB, m0, &a_full);
             }
             int s = 0; unsigned ph = 0;
-            for (int j = 0; j < n_tiles; ++j) {
-                const int jt = tile_of<ROT>(j, n_tiles);
-                for (int half = 0; half < BN / BNS; ++half)
-                    for (int kb = 0; kb < NKB; ++kb) {
-                        mb_wait(&b_empty[s], ph ^ 1u);           // the MMAs that read this slot have completed
-                        mb_expect(&b_full[s], 2 * BTILE_BYTES);
-                        tma_tile(B_st + (s * 2 + 0) * BTILE_BYTES, &tm_rhi, kb * KB, jt * BN + half * BNS, &b_full[s]);
-                        tma_tile(B_st + (s * 2 + 1) * BTILE_BYTES, &tm_rlo, kb * KB, jt * BN + half * BNS, &b_full[s]);
-                        if (++s == STAGES) { s = 0; ph ^= 1u; }
-                    }
-            }
+            for (int j = 0; j < n_tiles; ++j)
+                for (int kb = 0; kb < NKB; ++kb) {
+                    mb_wait(&b_empty[s], ph ^ 1u);               // the MMAs that read this slot have completed
+                    mb_expect(&b_full[s], 2 * BTILE_BYTES);
+                    tma_tile(B_st + (s * 2 + 0) * BTILE_BYTES, &tm_rhi, kb * KB, j * BN, &b_full[s]);
+                    tma_tile(B_st + (s * 2 + 1) * BTILE_BYTES, &tm_rlo, kb * KB, j * BN, &b_full[s]);
+                    if (++s == STAGES) { s = 0; ph ^= 1u; }
+                }
         }
     } else if (warp == 1) {
         // ===== MMA issuer (one thread issues; the warp stays converged on the barriers) =====
@@ -305,27 +286,25 @@ match_tc_kernel(const __grid_constant__ CUtensorMap tm_lhi, const __grid_constan
             const int buf = j & 1;
             mb_wait(&acc_empty[buf], ((unsigned)(j >> 1) & 1u) ^ 1u);   // the epilogue has drained this accumulator
             tc_fence_after();
-            for (int half = 0; half < BN / BNS; ++half) {
-                const unsigned d_tmem = tmem_base + (unsigned)(buf * BN + half * BNS);
-                for (int kb = 0; kb < NKB; ++kb) {
-                    mb_wait(&b_full[s], ph);
-                    tc_fence_after();
-                    if (lane == 0) {
-                        const uint64_t a_hi = umma_desc(A_hi + kb * TILE_BYTES), a_lo = umma_desc(A_lo + kb * TILE_BYTES);
-                        const uint64_t b_hi = umma_desc(B_st + (s * 2 + 0) * BTILE_BYTES), b_lo = umma_desc(B_st + (s * 2 + 1) * BTILE_BYTES);
+            const unsigned d_tmem = tmem_base + (unsigned)(buf * BN);
+            for (int kb = 0; kb < NKB; ++kb) {
+                mb_wait(&b_full[s], ph);
+                tc_fence_after();
+                if (lane == 0) {
+                    const uint64_t a_hi = umma_desc(A_hi + kb * TILE_BYTES), a_lo = umma_desc(A_lo + kb * TILE_BYTES);
+                    const uint64_t b_hi = umma_desc(B_st + (s * 2 + 0) * BTILE_BYTES), b_lo = umma_desc(B_st + (s * 2 + 1) * BTILE_BYTES);
 #pragma unroll
-                        for (int k8 = 0; k8 < KB / UMMA_K; ++k8) {
-                            const uint64_t adv = (uint64_t)(k8 * UMMA_K * 4 / 16);      // +32 bytes inside the swizzle span
-                            umma_tf32(d_tmem, a_hi + adv, b_hi + adv, (kb | k8) != 0 ? 1u : 0u, kIdesc);
-                            umma_tf32(d_tmem, a_hi + adv, b_lo + adv, 1u, kIdesc);
-                            umma_tf32(d_tmem, a_lo + adv, b_hi + adv, 1u, kIdesc);
-                        }
-                        umma_commit(&b_empty[s]);                // slot free once these MMAs have read it
-                        if (half == BN / BNS - 1 && kb == NKB - 1) umma_commit(&acc_full[buf]);
+                    for (int k8 = 0; k8 < KB / UMMA_K; ++k8) {
+                        const uint64_t adv = (uint64_t)(k8 * UMMA_K * 4 / 16);      // +32 bytes inside the swizzle span
+                        umma_tf32(d_tmem, a_hi + adv, b_hi + adv, (kb | k8) != 0 ? 1u : 0u, kIdesc);
+                        umma_tf32(d_tmem, a_hi + adv, b_lo + adv, 1u, kIdesc);
+                        umma_tf32(d_tmem, a_lo + adv, b_hi + adv, 1u, kIdesc);
                     }
-                    __syncwarp();
-                    if (++s == STAGES) { s = 0; ph ^= 1u; }
+                    umma_commit(&b_empty[s]);                    // slot free once these MMAs have read it
+                    if (kb == NKB - 1) umma_commit(&acc_full[buf]);
                 }
+                __syncwarp();
+                if (++s == STAGES) { s = 0; ph ^= 1u; }
             }
         }
     } else {
@@ -336,7 +315,7 @@ match_tc_kernel(const __grid_constant__ CUtensorMap tm_lhi, const __grid_constan
         const unsigned lane_base = tmem_base + ((unsigned)(q * 32) << 16);
         for (int j = 0; j < n_tiles; ++j) {
             const int buf = j & 1;
-            const int nb0 = tile_of<ROT>(j, n_tiles) * BN;
+            const int nb0 = j * BN;
             const float4* rn4 = reinterpret_cast<const float4*>(rnorm + nb0);
             // |b|^2 of the first group is on its way while the accumulator is still being written
             float4 rnA[8], rnB[8];
@@ -406,23 +385,11 @@ match_rerank_kernel(const ps_descriptor* __restrict__ l, int nl, const ps_descri
 
 } // namespace
 
-// POPSIFT_B200_MATCH=exact|tc overrides the automatic choice (A/B switch, cross-check)
-int match_choice(int flags)
-{
-    static const int env = [] {
-        const char* e = getenv("POPSIFT_B200_MATCH");
-        if (!e) return 0;
-        return e[0] == 'e' ? PS_MATCH_EXACT : e[0] == 't' ? PS_MATCH_TENSOR : 0;
-    }();
-    return flags ? flags : env;
-}
-
 int run_match(const ps_descriptor* l, int nl, const ps_descriptor* r, int nr, int32_t* out, int flags, cudaStream_t st,
               const char** err)
 {
     *err = nullptr;
     if (nl <= 0) return 0;
-    flags = match_choice(flags);
     // the tensor-core pass pays off from a few thousand pairs per left descriptor; below that (and for nr < 2, where
     // the reference's scan has its own corner cases) the CUDA-core kernel is the whole job
     const bool tensor = flags == PS_MATCH_TENSOR ? nr >= 1 : (flags == PS_MATCH_EXACT ? false : (nr >= 256 && (long long)nl * nr >= (1LL << 20)));
@@ -463,30 +430,15 @@ int run_match(const ps_descriptor* l, int nl, const ps_descriptor* r, int nr, in
     rhi = reinterpret_cast<float*>(ws + 2 * lb); rlo = reinterpret_cast<float*>(ws + 2 * lb + rb);
     rnorm = reinterpret_cast<float*>(ws + 2 * lb + 2 * rb);
     cand = reinterpret_cast<int32_t*>(ws + 2 * lb + 2 * rb + (size_t)nr_pad * 4);
-    // POPSIFT_B200_MATCH_RING = 128 | 64 | 128r | 64r: rows per B stage, r = every CTA starts at a different tile (A/B timing)
-    static const int ring_cfg = [] {
-        const char* e = getenv("POPSIFT_B200_MATCH_RING");
-        if (!e) return 0;
-        return (atoi(e) == 64 ? 1 : 0) | (strchr(e, 'r') ? 2 : 0);
-    }();
-    const int bns = (ring_cfg & 1) ? 64 : 128;
     CUtensorMap m_lhi, m_llo, m_rhi, m_rlo;
     const bool ok = make_tmap_2d(&m_lhi, lhi, 128, nl_pad, 512, KB, BM, true) && make_tmap_2d(&m_llo, llo, 128, nl_pad, 512, KB, BM, true) &&
-                    make_tmap_2d(&m_rhi, rhi, 128, nr_pad, 512, KB, bns, true) && make_tmap_2d(&m_rlo, rlo, 128, nr_pad, 512, KB, bns, true);
+                    make_tmap_2d(&m_rhi, rhi, 128, nr_pad, 512, KB, BN, true) && make_tmap_2d(&m_rlo, rlo, 128, nr_pad, 512, KB, BN, true);
     if (!ok) { cudaFreeAsync(ws, st); *err = "cuTensorMapEncodeTiled failed (matcher)"; return -1; }
     static_assert(TC_SMEM + 2048 <= 227 * 1024, "matcher shared memory");
     match_split_kernel<<<(nl_pad + 3) / 4, 128, 0, st>>>(l, nl, nl_pad, lhi, llo, nullptr);
     match_split_kernel<<<(nr_pad + 3) / 4, 128, 0, st>>>(r, nr, nr_pad, rhi, rlo, rnorm);
-    auto launch = [&](auto kern) {
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM);
-        kern<<<nl_pad / BM, TC_THREADS, TC_SMEM, st>>>(m_lhi, m_llo, m_rhi, m_rlo, rnorm, nl, n_tiles, cand);
-    };
-    switch (ring_cfg) {
-        case 1:  launch(match_tc_kernel<64, false>); break;
-        case 2:  launch(match_tc_kernel<128, true>); break;
-        case 3:  launch(match_tc_kernel<64, true>); break;
-        default: launch(match_tc_kernel<128, false>); break;
-    }
+    cudaFuncSetAttribute(match_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM);
+    match_tc_kernel<<<nl_pad / BM, TC_THREADS, TC_SMEM, st>>>(m_lhi, m_llo, m_rhi, m_rlo, rnorm, nl, n_tiles, cand);
     match_rerank_kernel<<<(nl + 3) / 4, 128, 0, st>>>(l, nl, r, nr, cand, out);
     cudaFreeAsync(ws, st);
     return 4;

@@ -21,13 +21,12 @@
 // 3x(box3, box3) smoothing, parabola refinement, peaks >= 0.8*best, theta = fma(2pi*bin, 1/36, -pi).
 #include "ps_internal.h"
 
-#include <cstdlib>
-
 namespace psb {
 
 namespace {
 
 constexpr int kWarps = 4;        // keypoints (warps) per CTA
+constexpr int kBatch = 4;        // window iterations evaluated together
 constexpr int kSlice = PS_ORI_SLICE;   // extrema per slice of the descriptor-index scan (ori_scatter_kernel)
 __device__ const float kPi  = 3.14159265358979323846f;
 __device__ const float kPi2 = 2.0f * 3.14159265358979323846f;
@@ -47,17 +46,13 @@ __device__ __forceinline__ int octave_prefix(const Counters* ct, const Consts& k
     return total;
 }
 
-// ATOMIC = true: histogram by shared float atomics like the reference (default); false: lane-private bins summed in
-// lane order (POPSIFT_B200_ORI_LANESUM=1; run-to-run deterministic by construction, ~20 % faster, not the reference's sums)
-template <bool ATOMIC, int WARPS, int BATCH>
-__global__ void __launch_bounds__(WARPS * 32)
+__global__ void __launch_bounds__(kWarps * 32)
 orientation_kernel(PyramidView pyr, Consts k, const InitialExtremum* __restrict__ iext_all, const InitialExtremum* __restrict__ iext_f,
                    ps_extremum* __restrict__ ext, int* __restrict__ slice_sum, Counters* ct)
 {
     const InitialExtremum* __restrict__ iext = ct->filtered ? iext_f : iext_all;
-    __shared__ float hist[ATOMIC ? 1 : WARPS][ATOMIC ? 1 : kOriBins * 33];     // lane-private bins (stride 33: conflict-free)
-    __shared__ float sm_a[WARPS][kOriBins];
-    __shared__ float sm_b[WARPS][kOriBins];
+    __shared__ float sm_a[kWarps][kOriBins];
+    __shared__ float sm_b[kWarps][kOriBins];
     __shared__ int   ps[kMaxOctaves + 1];
 
     if (threadIdx.x == 0) octave_prefix(ct, k, pyr.num_octaves, ps);
@@ -85,9 +80,7 @@ orientation_kernel(PyramidView pyr, Consts k, const InitialExtremum* __restrict_
         const int lvl = min(max(ie.lpos, 0), pyr.levels + 2);
         const float* pl = ov.gauss + (size_t)lvl * ov.plane;
 
-        float* Hp = hist[ATOMIC ? 0 : warp];
-        if (ATOMIC) { for (int b = lane; b < kOriBins; b += 32) A[b] = 0.0f; }
-        else        { for (int b = 0; b < kOriBins; ++b) Hp[b * 33 + lane] = 0.0f; }
+        for (int b = lane; b < kOriBins; b += 32) A[b] = 0.0f;
         __syncwarp();
 
         const float x = ie.xpos, y = ie.ypos, sig = ie.sigma;
@@ -110,17 +103,17 @@ orientation_kernel(PyramidView pyr, Consts k, const InitialExtremum* __restrict_
         // All lanes of an iteration reconverge before the atomic, like the reference's warp does.
         int xx = xmin + lane, yy = ymin;
         while (xx > xmax && wx > 0) { xx -= wx; ++yy; }
-        // BATCH iterations are evaluated together -- positions first, then all gradient loads (samples outside the window
+        // kBatch iterations are evaluated together -- positions first, then all gradient loads (samples outside the window
         // or the circle read the window's first pixel and are dropped afterwards), then the hypotf / atan2f / expf chains side
         // by side -- and their atomics issued in iteration order: per bin, the adds still arrive iteration by iteration, the
         // lanes of one iteration together.
         const float* safe = pl + (max(ymin, 1) * ov.pitch + max(xmin, 1));
-        for (int i0 = 0; i0 < loops; i0 += 32 * BATCH) {
-            int bidx[BATCH], sq[BATCH];
-            float weight[BATCH];
-            const float* p[BATCH];
+        for (int i0 = 0; i0 < loops; i0 += 32 * kBatch) {
+            int bidx[kBatch], sq[kBatch];
+            float weight[kBatch];
+            const float* p[kBatch];
 #pragma unroll
-            for (int u = 0; u < BATCH; ++u) {
+            for (int u = 0; u < kBatch; ++u) {
                 sq[u] = -1; p[u] = safe;
                 if (i0 + 32 * u + lane < loops) {
                     const float ddx = __fsub_rn((float)xx, x), ddy = __fsub_rn((float)yy, y);
@@ -133,14 +126,14 @@ orientation_kernel(PyramidView pyr, Consts k, const InitialExtremum* __restrict_
                     while (xx > xmax) { xx -= wx; ++yy; }
                 }
             }
-            float gdx[BATCH], gdy[BATCH];
+            float gdx[kBatch], gdy[kBatch];
 #pragma unroll
-            for (int u = 0; u < BATCH; ++u) {
+            for (int u = 0; u < kBatch; ++u) {
                 gdx[u] = __fsub_rn(__ldg(p[u] + 1), __ldg(p[u] - 1));
                 gdy[u] = __fsub_rn(__ldg(p[u] + ov.pitch), __ldg(p[u] - ov.pitch));
             }
 #pragma unroll
-            for (int u = 0; u < BATCH; ++u) {
+            for (int u = 0; u < kBatch; ++u) {
                 const float grad = hypotf(gdx[u], gdy[u]);
                 const float theta = atan2f(gdy[u], gdx[u]);
                 weight[u] = __fmul_rn(grad, expf(__fmul_rn((float)sq[u], factor)));
@@ -151,24 +144,12 @@ orientation_kernel(PyramidView pyr, Consts k, const InitialExtremum* __restrict_
                 bidx[u] = (sq[u] < 0 || b > kOriBins) ? -1 : b;
             }
 #pragma unroll
-            for (int u = 0; u < BATCH; ++u) {
-                if (ATOMIC) {
-                    __syncwarp();
-                    if (bidx[u] >= 0) atomicAdd(&A[bidx[u]], weight[u]);
-                } else if (bidx[u] >= 0) {
-                    Hp[bidx[u] * 33 + lane] += weight[u];
-                }
+            for (int u = 0; u < kBatch; ++u) {
+                __syncwarp();
+                if (bidx[u] >= 0) atomicAdd(&A[bidx[u]], weight[u]);
             }
         }
         __syncwarp();
-        if (!ATOMIC) {
-            for (int b = lane; b < kOriBins; b += 32) {
-                float sum = 0.0f;
-                for (int l = 0; l < 32; ++l) sum = __fadd_rn(sum, Hp[b * 33 + l]);
-                A[b] = sum;
-            }
-            __syncwarp();
-        }
         // 3 x (box3 ; box3), circular over 36 bins (reference s_orientation.cu:58-68,166-174)
         for (int it = 0; it < 3; ++it) {
             for (int b = lane; b < kOriBins; b += 32) {
@@ -328,17 +309,7 @@ int launch_orientation(const PyramidView& pyr, const Consts& k, const InitialExt
                        int* feat_to_ext, int* slice_sum, Counters* ct, cudaStream_t st)
 {
     // fixed grid: SMs x 8 resident CTAs of 4 warps; warps stride over the device-side count
-    static const bool lanesum = [] { const char* e = getenv("POPSIFT_B200_ORI_LANESUM"); return e && e[0] == '1'; }();
-    // experiments: POPSIFT_B200_ORI_WARPS=1 -> one warp per CTA like the reference's ori_par; POPSIFT_B200_ORI_GRID=n -> n CTAs
-    static const int one_warp = [] { const char* e = getenv("POPSIFT_B200_ORI_WARPS"); return e && e[0] == '1'; }();
-    static const int grid_env = [] { const char* e = getenv("POPSIFT_B200_ORI_GRID"); return e ? atoi(e) : 0; }();
-    const int grid = grid_env > 0 ? grid_env : sm_count() * 8;
-    static const int batch = [] { const char* e = getenv("POPSIFT_B200_ORI_BATCH"); return e ? atoi(e) : 4; }();
-    if (lanesum)         orientation_kernel<false, kWarps, 1><<<grid, kWarps * 32, 0, st>>>(pyr, k, iext, iext_f, ext, slice_sum, ct);
-    else if (one_warp)   orientation_kernel<true, 1, 1><<<grid_env > 0 ? grid_env : sm_count() * 32, 32, 0, st>>>(pyr, k, iext, iext_f, ext, slice_sum, ct);
-    else if (batch == 2) orientation_kernel<true, kWarps, 2><<<grid, kWarps * 32, 0, st>>>(pyr, k, iext, iext_f, ext, slice_sum, ct);
-    else if (batch == 4) orientation_kernel<true, kWarps, 4><<<grid, kWarps * 32, 0, st>>>(pyr, k, iext, iext_f, ext, slice_sum, ct);
-    else                 orientation_kernel<true, kWarps, 1><<<grid, kWarps * 32, 0, st>>>(pyr, k, iext, iext_f, ext, slice_sum, ct);
+    orientation_kernel<<<sm_count() * 8, kWarps * 32, 0, st>>>(pyr, k, iext, iext_f, ext, slice_sum, ct);
     ori_scatter_kernel<<<k.ext_capacity / kSlice + 1, kSlice, 0, st>>>(pyr.num_octaves, k, ext, feat_to_ext, slice_sum, ct);
     return 2;
 }

@@ -65,7 +65,7 @@ PSB_HD bool locate(const Partition& p, int b, int H, int Q, int& strip, int& ys,
     return ys < H;
 }
 
-inline Partition make_partition(int W, int H, int TW, int Q, int slots, bool uniform)
+inline Partition make_partition(int W, int H, int TW, int Q, int slots)
 {
     Partition p;
     const int S = (W + TW - 1) / TW;
@@ -82,7 +82,7 @@ inline Partition make_partition(int W, int H, int TW, int Q, int slots, bool uni
     p.uh = u;
     p.nh = (C + u - 1) / u;
     p.nl = p.nh; p.ul = u; p.heavy = S; p.pad = 0;
-    if (!uniform && u - 1 >= 4 && S * p.nh < slots) {
+    if (u - 1 >= 4 && S * p.nh < slots) {
         const int nl = (C + u - 2) / (u - 1);
         if (nl > p.nh) {
             int x = (slots - S * p.nh) / (nl - p.nh);      // light strips that fit in the spare slots

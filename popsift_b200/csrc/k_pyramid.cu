@@ -381,10 +381,6 @@ int level0_plan(int w, int h, int W, int H, float shift, int R)
     std::lock_guard<std::mutex> lk(mu);
     auto it = cache.find(key);
     if (it != cache.end()) return it->second;
-    if (const char* e = getenv("POPSIFT_B200_LEVEL0")) {           // A/B: force one evaluation ("shared" is unchecked)
-        if (!strcmp(e, "pertap")) return cache[key] = LEVEL0_PER_TAP;
-        if (!strcmp(e, "shared")) return cache[key] = LEVEL0_SHARED;
-    }
     bool shared = true;
     for (int X = 0; X < W && shared; ++X) {
         const float cx = tex_coord_centre(X, shift, W);

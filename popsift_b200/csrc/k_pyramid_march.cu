@@ -28,7 +28,6 @@
 #include "tma_util.h"
 
 #include <cstdint>
-#include <cstdlib>
 #include <mutex>
 #include <set>
 #include <utility>
@@ -376,11 +375,6 @@ march_level_kernel(const __grid_constant__ CUtensorMap tmap, const float* __rest
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         if (CAND) s_cand_n = 0;
     }
-    // programmatic dependent launch: everything above overlaps the previous grid's tail; its planes are complete and
-    // visible after the wait.  The next grid may be scheduled as soon as every CTA of this one has passed this point
-    // (it waits for our completion in the same way).
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     __syncthreads();
     if (!edge) march_body<R, false, NEXT, CAND>(smem, full, &tmap, src, dst, dog, next0, W, H, pitch, next_pitch, x0, ys, ye, taps, sink, &s_cand_n);
     else       march_body<R, true, NEXT, CAND>(smem, full, &tmap, src, dst, dog, next0, W, H, pitch, next_pitch, x0, ys, ye, taps, sink, &s_cand_n);
@@ -597,32 +591,9 @@ march_level0x2_kernel(const uint8_t* __restrict__ img, size_t img_pitch, int w, 
 
 // ---- launch helpers ---------------------------------------------------------------------------
 
-// POPSIFT_B200_UNIFORM=1 keeps every strip at the same segment length (A/B timing)
-bool uniform_choice()
-{
-    static const bool v = [] { const char* e = getenv("POPSIFT_B200_UNIFORM"); return e && e[0] == '1'; }();
-    return v;
-}
-
 Partition make_partition(int W, int H, int slots = 0)     // one wave: SMs x 4 resident CTAs (592 on B200)
 {
-    return psb::make_partition(W, H, TW, Q, slots > 0 ? slots : 4 * sm_count(), uniform_choice());
-}
-
-// resident CTAs of the exact-2x level-0 kernel (POPSIFT_B200_L0SLOTS overrides, A/B timing)
-int level0_slots()
-{
-    static const int v = [] { const char* e = getenv("POPSIFT_B200_L0SLOTS"); const int n = e ? atoi(e) : 0; return n; }();
-    return v > 0 ? v : 6 * sm_count();
-}
-
-// POPSIFT_B200_PDL=1 launches the level kernels with programmatic dependent launch.  Off by default: measured
-// 0.794 ms (on) vs 0.777 ms (off) for the 4K pyramid -- the early-launched CTAs of the next level take the slots the
-// side stream's ready kernels (levels L+1, L+2 of the previous octave) would otherwise run in.
-bool pdl_choice()
-{
-    static const bool v = [] { const char* e = getenv("POPSIFT_B200_PDL"); return e && e[0] == '1'; }();
-    return v;
+    return psb::make_partition(W, H, TW, Q, slots > 0 ? slots : 4 * sm_count());
 }
 
 template <int R, bool NEXT, bool CAND>
@@ -632,16 +603,9 @@ int launch_march(const Partition& part, const float* src, float* dst, float* dog
     ensure_smem(march_level_kernel<R, NEXT, CAND>, Geo<R>::smem, true);
     CUtensorMap map;
     if (!make_tmap_2d(&map, src, o.w, o.h, (size_t)o.pitch * sizeof(float), Geo<R>::SWP, Q, false)) return -2;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(part.B); cfg.blockDim = dim3(NT); cfg.dynamicSmemBytes = Geo<R>::smem; cfg.stream = st;
-    // programmatic dependent launch: the next level's CTAs are scheduled while this grid drains and run their
-    // prologue (partition lookup, mbarrier init); they touch the planes only after griddepcontrol.wait
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = pdl_choice() ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, march_level_kernel<R, NEXT, CAND>, map, src, dst, dog, next0, o.w, o.h, o.pitch, next_pitch,
-                              part, t, sink) == cudaSuccess ? 1 : -2;
+    march_level_kernel<R, NEXT, CAND><<<part.B, NT, Geo<R>::smem, st>>>(map, src, dst, dog, next0, o.w, o.h, o.pitch, next_pitch,
+                                                                        part, t, sink);
+    return 1;
 }
 
 template <int R>
@@ -667,7 +631,8 @@ int run_march0(const PIX* img, size_t img_pitch, int w, int h, float shift, cons
         const bool x2 = plan == LEVEL0_IDEAL_X2 && shift == 1.0f && o0.w == 2 * w && o0.h == 2 * h && (img_pitch & 3) == 0 &&
                         (reinterpret_cast<uintptr_t>(img) & 3) == 0;
         if (x2) {
-            const Partition part = make_partition(o0.w, o0.h, level0_slots());
+            // one wave: 26 KB of shared memory per CTA allows 6 resident CTAs per SM
+            const Partition part = make_partition(o0.w, o0.h, 6 * sm_count());
             ensure_smem(march_level0x2_kernel<R>, Geo0<R>::smem, true);
             march_level0x2_kernel<R><<<part.B, NT, Geo0<R>::smem, st>>>(img, img_pitch, w, h, o0.gauss, o0.w, o0.h, o0.pitch,
                                                                         part, dd, inc0);

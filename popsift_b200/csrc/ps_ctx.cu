@@ -169,13 +169,6 @@ int build_view(ps_ctx* ctx, Slot& s, int w, int h)
     return PS_OK;
 }
 
-// POPSIFT_B200_FORK=0 keeps the whole pyramid on one stream (A/B switch)
-bool fork_choice()
-{
-    static const bool v = [] { const char* e = getenv("POPSIFT_B200_FORK"); return !(e && e[0] == '0'); }();
-    return v;
-}
-
 // device pitch of the 8-bit input image: rows start 4-byte aligned (the level-0 kernel stages them with
 // 4-byte cp.async)
 static inline size_t u8_pitch(int w) { return ((size_t)w + 3) & ~(size_t)3; }
@@ -199,7 +192,7 @@ static bool level_sink(ps_ctx* ctx, Slot& s, int o, int l, CandSink& cs)
 int run_pyramid(ps_ctx* ctx, Slot& s)
 {
     const int L = ctx->levels;
-    const bool fork = fork_choice() && s.num_octaves > 1;
+    const bool fork = s.num_octaves > 1;
     const bool direct = ctx->cfg.scaling_mode == PS_SCALE_DIRECT;
     int n = 0, r;
     // the pyramid kernels report the threshold-passing DoG samples when every scanned level runs on the

@@ -320,7 +320,6 @@ def test_fallback_paths_give_the_same_counts():
     assert base[0] > 1000
     assert _counts_in_subprocess({"POPSIFT_B200_DENSE_SCAN": "1"}, w, h) == base
     assert _counts_in_subprocess({"POPSIFT_B200_TILE_KERNELS": "1"}, w, h) == base
-    assert _counts_in_subprocess({"POPSIFT_B200_UNIFORM": "1", "POPSIFT_B200_FORK": "0"}, w, h) == base
     # a slot whose extremum / descriptor buffers are far too small grows them on demand and re-runs the orientation
     # and descriptor stages (reference Pyramid::reallocExtrema, sift_pyramid.cu:179-209): same result, nothing truncated
     assert _counts_in_subprocess({"POPSIFT_B200_INIT_CAP": "100"}, w, h) == base

@@ -373,7 +373,9 @@ def test_level0_plan_follows_the_texture_coordinate_model():
 def test_shipped_sass_uses_tma_and_tcgen05():
     """The claims of DESIGN.md about the hardware paths, checked on the built library itself (cuobjdump, no GPU needed):
     every column-marching level kernel stages its rows with the TMA unit (UTMALDG + mbarrier SYNCS), its column pass is packed
-    FFMA2, and the matcher issues tcgen05 MMAs (UTCHMMA) with TMEM loads (LDTM)."""
+    FFMA2, and the matcher issues tcgen05 MMAs (UTCHMMA) with TMEM loads (LDTM).  Only the variants that run are shipped: one
+    orientation kernel, one tensor-core matcher, one candidate extrema kernel per SIFT mode, and level kernels without
+    programmatic-dependent-launch instructions (ACQBULK / PREEXIT)."""
     import shutil
     import sys as _sys
     if shutil.which("cuobjdump") is None:
@@ -389,8 +391,34 @@ def test_shipped_sass_uses_tma_and_tcgen05():
     for n, c in level.items():
         assert c["UTMALDG"] > 0 and c["SYNCS"] > 0 and c["FFMA2"] > 0, n
         assert c["LDGSTS"] == 0, n                       # no cp.async staging left in the level kernels
+        assert c["ACQBULK"] == 0 and c["PREEXIT"] == 0, n
     tc = {n: c for n, c in k.items() if "match_tc_kernel" in n}
-    assert tc and all(c["UTCHMMA"] > 0 and c["LDTM"] > 0 and c["UTMALDG"] > 0 for c in tc.values())
+    assert len(tc) == 1 and all(c["UTCHMMA"] > 0 and c["LDTM"] > 0 and c["UTMALDG"] > 0 for c in tc.values())
+    assert sum("orientation_kernel" in n for n in k) == 1
+    assert sum("cand_extrema_kernel" in n for n in k) == 3
+
+
+def test_runtime_switches_are_the_documented_ones():
+    """The POPSIFT_B200_* environment variables the library reads (getenv under popsift_b200/csrc) are exactly the ones
+    INTEGRATION.md section 5 lists, apart from the two that Python code reads: POPSIFT_B200_LIB (api.py) and
+    POPSIFT_BENCH_SLOTS (bench.py)."""
+    read = set()
+    for dp, _, fs in os.walk(os.path.join(ROOT, "popsift_b200", "csrc")):
+        for f in fs:
+            with open(os.path.join(dp, f), errors="replace") as fh:
+                read |= set(re.findall(r'getenv\("(POPSIFT_B200_\w+)"\)', fh.read()))
+    with open(os.path.join(ROOT, "INTEGRATION.md")) as fh:
+        sec = fh.read().split("\n## 5.")[1].split("\n## ")[0]
+    listed = set()
+    for ln in sec.splitlines():
+        if ln.startswith("| `"):
+            listed |= set(re.findall(r"`(POPSIFT_\w+?)[=`]", ln.split(" | ")[0]))
+    python_side = {"POPSIFT_B200_LIB": "popsift_b200/api.py", "POPSIFT_BENCH_SLOTS": "bench.py"}
+    for name, path in python_side.items():
+        with open(os.path.join(ROOT, path)) as fh:
+            assert name in fh.read(), (name, path)
+    assert read, "no getenv calls found"
+    assert listed - set(python_side) == read, (sorted(listed - set(python_side) - read), sorted(read - listed))
 
 
 def test_print_gauss_tables_text():

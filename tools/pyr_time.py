@@ -27,7 +27,7 @@ def timeit(fn, n=10, warm=3):
     return statistics.median(ts)
 t = timeit(lambda: L.ps_run_pyramid_only(ctx, 0))
 sumwh = sum(w * h for w, h in geo)
-print("env MINB=%s TILE=%s" % (os.environ.get("POPSIFT_B200_MINB"), os.environ.get("POPSIFT_B200_TILE_KERNELS")))
+print("env TILE=%s" % os.environ.get("POPSIFT_B200_TILE_KERNELS"))
 print("pyramid stage: %.3f ms  -> %.0f GB/s algorithmic (68 B/px, %d px)" % (t, 68 * sumwh / t / 1e6, sumwh))
 for o in range(min(2, len(geo))):
     for l in range(0 if o == 0 else 1, 6):
